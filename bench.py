@@ -265,6 +265,9 @@ def main():
     ap.add_argument("--workload", default="walk", choices=["walk", "mixed"],
                     help="walk: BASELINE configs[1] (walking-gait states); mixed: configs[2] (25 %% stand / 75 %% walk, randomized)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step of the device and end-to-end legs as DIR/<name>.npy "
+                         "(with several GPUs: rank 0's robots)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -379,6 +382,8 @@ def main():
     barrier()
     e2e_s = time.perf_counter() - t0
     assert (interface.status_code(out_s[:B]) == 0).all(), "non-converged instances in the end-to-end leg"
+    # the end-to-end leg's result arrays are reused below: keep what its last timed step returned
+    e2e_w_last, e2e_s_last = np.array(out_w[:B]), np.array(out_s[:B])
     # after the timed region: what the gather delivered (every rank's slice, on this device) against the oracle
     parity = None
     if world > 1:
@@ -411,6 +416,21 @@ def main():
     st = d_st[(W + K - 1) % ring].cpu().numpy()
     assert (interface.status_code(st) == 0).all(), "non-converged instances in the timed region"
     iters = interface.status_iters(st)
+    if args.dump_outputs and rank == 0:
+        # inputs are seeded (scenarios.make_batch), so two builds run with the same arguments can be compared array for array
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dump = {"device_wrench": d_out[(W + K - 1) % ring].cpu().numpy(),
+                "device_status_code": interface.status_code(st), "device_status_iters": iters,
+                "e2e_wrench": e2e_w_last, "e2e_status_code": interface.status_code(e2e_s_last),
+                "e2e_status_iters": interface.status_iters(e2e_s_last)}
+        rows = np.arange(B)
+        row_bytes = sum(int(np.prod(np.shape(a)[1:])) * (8 if np.asarray(a).dtype == np.float64 else 4) for a in dump.values()) + 8
+        if B * row_bytes > 64 << 20:  # at most 64 MB: a fixed, seeded sample of the robots
+            rows = np.sort(np.random.default_rng(0).choice(B, (64 << 20) // row_bytes, replace=False))
+        for name, a in dump.items():
+            a = np.asarray(a)[rows]
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+        np.save(os.path.join(args.dump_outputs, "robot_index.npy"), rows.astype(np.float64))
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()

@@ -823,11 +823,6 @@ HMPC_EXTERNC int hmpc_prepare_device(hmpc_ctx* c, const hmpc_state_t* d_states, 
 {
   if (!c || !d_states || !d_records || B < 0) { g_err = "hmpc_prepare_device: bad argument"; return HMPC_ERR_ARG; }
   if (B == 0) return HMPC_OK;
-  if (g_fail_next_solves > 0) {
-    g_fail_next_solves--;
-    g_err = "injected failure (hmpc_debug_fail_next_solves)";
-    return HMPC_ERR_CUDA;
-  }
   CK(cudaSetDevice(c->device));
   hmpc::hmpc_prepare_kernel<<<(B + 63) / 64, 64, 0, static_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const unsigned char*>(d_states), B, c->horizon, dtMPC,
@@ -969,6 +964,11 @@ static int solve_batch_impl(hmpc_ctx* c, const update_data_t* in, const hmpc_sta
     return HMPC_ERR_ARG;
   }
   if (B == 0) return HMPC_OK;
+  if (g_fail_next_solves > 0) {
+    g_fail_next_solves--;
+    g_err = "injected failure (hmpc_debug_fail_next_solves)";
+    return HMPC_ERR_CUDA;
+  }
   CK(cudaSetDevice(c->device));
   const size_t nw = (size_t)12 * c->horizon;
   // pipeline over chunks: the host packs chunk k+1 while the GPU copies/solves chunk k, and converts the

@@ -8,7 +8,7 @@ in SolverMPC.cpp); the fp64-assembly oracle quantifies what fp32 assembly costs 
 import numpy as np
 import pytest
 
-from conftest import rel_err
+from conftest import reference_solve, rel_err
 from hector_simulation_b200 import interface, scenarios
 
 pytestmark = pytest.mark.gpu
@@ -33,8 +33,6 @@ def _step(state, u0, feet, dt):
 
 
 def test_closed_loop_ticks_match_oracle(oracle):
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
     from oracle import qp_dual_active_set as G
 
     # The harness has no swing-leg foot placement (out of scope), so single-support robots tip over after
@@ -62,7 +60,7 @@ def test_closed_loop_ticks_match_oracle(oracle):
         wrench, status = mpc.solve_batch(recs)
         assert (interface.status_code(status) == 0).all(), (t, np.bincount(interface.status_code(status)))
         idx = np.arange(t % 4, B, 4)
-        ref, info = oracle.solve_batch(recs[idx], setup)
+        ref, info = reference_solve(oracle, recs[idx], setup)
         assert (info[:, 0] == 0).all()
         e = rel_err(wrench[idx], ref, 12)
         worst = max(worst, float(e.max()))
@@ -78,7 +76,7 @@ def test_closed_loop_ticks_match_oracle(oracle):
             assert rel_err(wrench[idx[k]][None], full[None], 12)[0] < 2e-6
             refereed += 1
         if t % 6 == 0:
-            ref64, _ = oracle.solve_batch(recs[idx], setup, True)
+            ref64, _ = reference_solve(oracle, recs[idx], setup, assembly_fp64=True)
             worst64 = max(worst64, float(rel_err(wrench[idx], ref64, 12).max()))
         for i in range(B):
             states[i] = _step(states[i], wrench[i, :12], feet[i], scenarios.DT_MPC)

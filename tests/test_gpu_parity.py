@@ -10,7 +10,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import load_golden, rel_err
+from conftest import load_golden, qpoases_sample, reference_solve, rel_err
 from hector_simulation_b200 import interface, scenarios
 
 pytestmark = pytest.mark.gpu
@@ -145,14 +145,12 @@ def test_reference_boundary_single_robot(torch_cuda):
     assert all(sol2[3 * leg_swing + c] == 0.0 and sol2[6 + 3 * leg_swing + c] == 0.0 for c in range(3))
 
 
-def test_full_size_configs_vs_live_oracle(torch_cuda, oracle):
-    """BASELINE configs[1] (B=1024 walking) in full; configs[2] (B=8192 mixed) on a strided sample of the oracle."""
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
-    setup = oracle.make_setup(10)
+def test_full_size_configs_vs_live_oracle(torch_cuda):
+    """BASELINE configs[1] (B=1024 walking) in full; configs[2] (B=8192 mixed) on a strided sample, against qpOASES'
+    recorded optimum of the same seeded inputs."""
     recs, _ = scenarios.make_batch(2, 1024, horizon=10)
     w, st = _solve(recs, 10)
-    ref, info = oracle.solve_batch(recs, setup)
+    ref, _ = qpoases_sample("full_cfg2", recs)
     assert (interface.status_code(st) == 0).all()
     e = rel_err(w, ref, 12)
     assert e.max() < TOL and np.median(e) < 1e-6
@@ -160,7 +158,7 @@ def test_full_size_configs_vs_live_oracle(torch_cuda, oracle):
     w3, st3 = _solve(recs3, 10)
     assert (interface.status_code(st3) == 0).all()
     idx = np.arange(0, 8192, 16)
-    ref3, _ = oracle.solve_batch(recs3[idx], setup)
+    ref3, _ = qpoases_sample("full_cfg3", recs3[idx])
     assert rel_err(w3[idx], ref3, 12).max() < TOL
     assert rel_err(w3[idx], ref3).max() < TOL
 
@@ -228,9 +226,7 @@ def test_edge_cases(torch_cuda):
     mpc.close()
 
 
-def test_edge_cases_vs_oracle(torch_cuda, oracle):
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
+def test_edge_cases_vs_oracle(torch_cuda):
     N = 10
     rng = np.random.default_rng(5)
     recs = []
@@ -240,8 +236,8 @@ def test_edge_cases_vs_oracle(torch_cuda, oracle):
         recs.append(scenarios.to_record(b, N))
     recs = np.array(recs)
     w, s = _solve(recs, N)
-    ref, info = oracle.solve_batch(recs, oracle.make_setup(N))
-    assert (interface.status_code(s) == 0).all() and (info[:, 0] == 0).all()
+    ref, rc = qpoases_sample("ragged48", recs)
+    assert (interface.status_code(s) == 0).all() and (rc == 0).all()
     assert rel_err(w, ref).max() < TOL
     assert (w[ref == 0.0] == 0.0).all()
 
@@ -305,24 +301,23 @@ def test_stress_large_perturbations_all_converge(torch_cuda, oracle):
     codes = np.bincount(interface.status_code(st), minlength=5)
     assert codes[1:].sum() == 0, codes
     assert np.isfinite(w).all()
-    if oracle.has_qpoases():
-        from oracle import qp_dual_active_set as G
+    from oracle import qp_dual_active_set as G
 
-        idx = np.arange(0, B, 32)
-        setup = oracle.make_setup(N)
-        ref, info = oracle.solve_batch(recs[idx], setup)
-        good = info[:, 0] == 0
-        e0, ef = rel_err(w[idx], ref, 12), rel_err(w[idx], ref)
-        assert e0[good].max() < 1e-4 and np.median(e0[good]) < 1e-5   # first-step wrench: the contract
-        # whole horizon: far from the nominal regime qpOASES itself is up to ~1e-4 away from the exact optimum
-        # (termination tolerance 2.2e-7 in homotopy length); the three largest gaps are refereed in fp64
-        for k in np.argsort(-np.where(good, ef, 0))[:3]:
-            Q = oracle.reduced_qp(recs[idx[k]], setup)
-            x, inf = G.solve(Q["H"], Q["g"], Q["A"], Q["lb"], Q["ub"], tol=1e-12, max_iter=3000)
-            full = np.zeros(12 * N)
-            full[Q["var_ind"]] = x
-            assert inf["status"] == 0 and rel_err(w[idx[k]][None], full[None])[0] < 1e-6
-        assert ef[good].max() < 3e-4
+    idx = np.arange(0, B, 32)
+    setup = oracle.make_setup(N)
+    ref, info = reference_solve(oracle, recs[idx], setup)
+    good = info[:, 0] == 0
+    e0, ef = rel_err(w[idx], ref, 12), rel_err(w[idx], ref)
+    assert e0[good].max() < 1e-4 and np.median(e0[good]) < 1e-5   # first-step wrench: the contract
+    # whole horizon: far from the nominal regime qpOASES itself is up to ~1e-4 away from the exact optimum
+    # (termination tolerance 2.2e-7 in homotopy length); the three largest gaps are refereed in fp64
+    for k in np.argsort(-np.where(good, ef, 0))[:3]:
+        Q = oracle.reduced_qp(recs[idx[k]], setup)
+        x, inf = G.solve(Q["H"], Q["g"], Q["A"], Q["lb"], Q["ub"], tol=1e-12, max_iter=3000)
+        full = np.zeros(12 * N)
+        full[Q["var_ind"]] = x
+        assert inf["status"] == 0 and rel_err(w[idx[k]][None], full[None])[0] < 1e-6
+    assert ef[good].max() < 3e-4
 
 
 def test_in_place_mode_equals_staged_path():
@@ -443,14 +438,12 @@ def test_horizon_sweep_batch_4096(torch_cuda, oracle, N):
     w, st = mpc.solve_batch(recs, strict=False)
     mpc.close()
     assert (interface.status_code(st) == 0).all(), np.bincount(interface.status_code(st))
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
     from oracle import qp_dual_active_set as G
 
     idx = np.arange(3, B, 64 if N <= 10 else 128)
     setup = oracle.make_setup(N)
-    ref, info = oracle.solve_batch(recs[idx], setup)
-    good = info[:, 0] == 0
+    ref, rc = qpoases_sample("sweep_h%d" % N, recs[idx])
+    good = rc == 0
     e0, ef = rel_err(w[idx], ref, 12), rel_err(w[idx], ref)
     assert e0[good].max() < 1e-4 and np.median(e0[good]) < 1e-5
     refereed = 0

@@ -423,10 +423,10 @@ def test_solve_kernel_source_has_no_data_races(emul, tmp_path):
         assert r.returncode == (0 if key.startswith("h10_x8") else 1), (key, r.returncode, r.stdout)   # lying: reported, not solved
 
 
-def test_solve_kernel_source_edge_cases(emul, oracle):
+def test_solve_kernel_source_edge_cases(emul):
     """The contact-schedule edge cases of the -m gpu suite on the kernel source: no foot in contact over the whole horizon
-    (everything eliminated), flight then double support, and arbitrary ragged schedules against the live oracle."""
-    from conftest import rel_err
+    (everything eliminated), flight then double support, and arbitrary ragged schedules against qpOASES' recorded optimum."""
+    from conftest import qpoases_sample, rel_err
 
     N = 10
     b = scenarios.stand_inputs(N)
@@ -443,20 +443,17 @@ def test_solve_kernel_source_edge_cases(emul, oracle):
     assert (interface.status_code(st) == 0).all()
     assert (w[0] == 0).all()
     assert (w[1, :48] == 0).all() and np.abs(w[1, 48:]).max() > 1
-    if oracle.has_qpoases():
-        ref, info = oracle.solve_batch(recs, oracle.make_setup(N))
-        assert (info[:, 0] == 0).all()
-        assert rel_err(w[1:], ref[1:]).max() < 5e-5
-        assert (w[ref == 0.0] == 0.0).all()
+    ref, rc = qpoases_sample("edges8", recs)
+    assert (rc == 0).all()
+    assert rel_err(w[1:], ref[1:]).max() < 5e-5
+    assert (w[ref == 0.0] == 0.0).all()
 
 
-def test_solve_kernel_source_working_sets_beyond_the_column_cache(emul, oracle):
+def test_solve_kernel_source_working_sets_beyond_the_column_cache(emul):
     """Class 0 caches H^-1 a_j for its first N + 4 working-set slots and holds up to 2N + 4 rows: walking robots whose optimum
     has more active rows than the cache (15, 16 and 19 here; ~1 % of the configs[1] batches) stay in class 0 — their primal
     steps go through a full H^-1 product for the slots beyond the cache — instead of being handed to the slower class 1."""
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
-    from conftest import rel_err
+    from conftest import qpoases_sample, rel_err
 
     N = 10
     picks = ((1000, [780, 20]), (4000, [217]))
@@ -465,8 +462,8 @@ def test_solve_kernel_source_working_sets_beyond_the_column_cache(emul, oracle):
     assert launched.tolist() == [3, 0, 0]                              # nobody escalates
     assert (interface.status_code(st) == 0).all()
     assert sorted(interface.status_nactive(st).tolist()) == [15, 16, 19]
-    ref, info = oracle.solve_batch(recs, oracle.make_setup(N))
-    assert (info[:, 0] == 0).all() and rel_err(w, ref, 12).max() < 5e-6 and rel_err(w, ref).max() < 5e-5
+    ref, rc = qpoases_sample("column_cache", recs)
+    assert (rc == 0).all() and rel_err(w, ref, 12).max() < 5e-6 and rel_err(w, ref).max() < 5e-5
 
 
 def test_solve_kernel_source_is_insensitive_to_its_two_tolerances(emul):
@@ -523,10 +520,8 @@ def test_closed_loop_of_kernel_sources(emul, oracle):
     """hmpc_rollout_device's tick — data-preparation kernel -> classification + solve kernels -> advance kernel — with all
     three kernels' sources chained on the host, against the same loop driven from the host (host mirror of the preparation,
     the same solve, numpy mirror of the advance step: the comparison tests/test_rollout.py makes on the GPU), with qpOASES
-    checking every tick's wrench."""
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
-    from conftest import rel_err
+    (or, where it is not built, the exact fp64 referee of the same QPs) checking every tick's wrench."""
+    from conftest import reference_solve, rel_err
     from test_rollout import _host_prepared, _walkers
 
     N, B, T = 10, 3, 8
@@ -552,7 +547,7 @@ def test_closed_loop_of_kernel_sources(emul, oracle):
         # host-driven loop
         recs = _host_prepared(states, N)
         w_h, st_h = solve(np.ascontiguousarray(interface.pack_records(recs, N)))
-        q, info = oracle.solve_batch(recs, setup)
+        q, info = reference_solve(oracle, recs, setup)
         assert (info[:, 0] == 0).all() and rel_err(w_h.astype(np.float64), q, 12).max() < 5e-5
         scenarios.advance_numpy(states, loop, w_h, st_h, N)
         # the kernels' loop

@@ -55,13 +55,15 @@ def test_torque_oracle_stand_is_symmetric(oracle):
 
 @pytest.mark.gpu
 def test_fused_torque_epilogue_vs_oracle(oracle):
+    from conftest import qpoases_sample
     from hector_simulation_b200 import interface
 
     recs, inputs = scenarios.make_batch(3, 256, horizon=10, seed=31)
     mpc = interface.BatchedMPC(256, 10)
     w, tau, st = mpc.solve_batch_torques(recs)
     assert (interface.status_code(st) == 0).all()
-    ref_w, _ = oracle.solve_batch(recs, oracle.make_setup(10)) if oracle.has_qpoases() else (w, None)
+    ref_w, rc = qpoases_sample("torques256", recs)             # qpOASES' first-step wrenches of the same records
+    assert (rc == 0).all()
     rB = np.array([b["rBody"] for b in inputs])
     ql = np.array([b["q_leg"] for b in inputs])
     contact = np.array([b["gait"][:2] for b in inputs])

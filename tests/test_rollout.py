@@ -4,7 +4,7 @@ advance per tick, no host in the loop) against (1) the numpy mirror of the advan
 import numpy as np
 import pytest
 
-from conftest import rel_err
+from conftest import reference_solve, rel_err
 from hector_simulation_b200 import interface, scenarios
 from test_state_prepare import _host_prepared
 
@@ -34,16 +34,15 @@ def test_gait_advance_matches_gait_class():
 
 
 def test_numpy_loop_with_oracle_keeps_walkers_upright(oracle):
-    """The loop semantics (plant, touch-down placement, set-point integration) with qpOASES as the solver."""
-    if not oracle.has_qpoases():
-        pytest.skip("oracle/_ref without qpOASES")
+    """The loop semantics (plant, touch-down placement, set-point integration) with qpOASES (or, where it is not built,
+    the exact fp64 referee of the same QPs) as the solver."""
     states, loop = _walkers(4)
     cmd = states["state_des"][:, 2].copy()
     x0 = states["position"][:, 0].copy()
     setup = oracle.make_setup(N)
     T = 40
     for t in range(T):
-        q, info = oracle.solve_batch(_host_prepared(states, N), setup)
+        q, info = reference_solve(oracle, _host_prepared(states, N), setup)
         assert (info[:, 0] == 0).all()
         scenarios.advance_numpy(states, loop, q, (info[:, 1].astype(np.int32) << 8), N)
     assert (np.abs(states["position"][:, 2] - 0.56) < 0.03).all() and (np.abs(states["rpy"][:, :2]) < 0.05).all()
@@ -89,17 +88,16 @@ def test_device_rollout_matches_host_driven_loop(oracle):
     assert (np.abs(dev_states["position"][:, 2] - 0.56) < 0.03).all()
 
     # (2) the records the device loop logged, solved by the oracle (strided sample), against the logged wrenches
-    if oracle.has_qpoases():
-        setup = oracle.make_setup(N)
-        worst = 0.0
-        for t in range(0, T, 4):
-            idx = np.arange(t % 8, B, 8)
-            recs = interface.unpack_records(rlog[t][idx], N)
-            ref, info = oracle.solve_batch(recs, setup)
-            assert (info[:, 0] == 0).all()
-            worst = max(worst, float(rel_err(wlog[t][idx].astype(np.float64), ref[:, :12], 12).max()))
-        print("device rollout vs oracle on logged records: worst rel err %.3e; vs host-driven loop %.3e" % (worst, worst_w))
-        assert worst < 1e-4, worst
+    setup = oracle.make_setup(N)
+    worst = 0.0
+    for t in range(0, T, 4):
+        idx = np.arange(t % 8, B, 8)
+        recs = interface.unpack_records(rlog[t][idx], N)
+        ref, info = reference_solve(oracle, recs, setup)
+        assert (info[:, 0] == 0).all()
+        worst = max(worst, float(rel_err(wlog[t][idx].astype(np.float64), ref[:, :12], 12).max()))
+    print("device rollout vs oracle on logged records: worst rel err %.3e; vs host-driven loop %.3e" % (worst, worst_w))
+    assert worst < 1e-4, worst
     mpc.close()
 
 
@@ -139,18 +137,17 @@ def test_config5_200_ticks_on_device(oracle):
     wc = rel_err(sel_w.reshape(-1, 12), w_cold[:, :12], 12)
     print("config 5: warm-started loop vs cold solve of the same records: worst rel err %.3e" % wc.max())
     assert wc.max() < 1e-6   # float32 output resolution; the optimum is the same point
-    if oracle.has_qpoases():
-        setup = oracle.make_setup(N)
-        ref, info = oracle.solve_batch(recs, setup)
-        ok = info[:, 0] == 0
-        e32 = rel_err(sel_w.reshape(-1, 12)[ok], ref[ok][:, :12], 12)
-        ref64, info64 = oracle.solve_batch(recs, setup, True)
-        ok64 = ok & (info64[:, 0] == 0)
-        e64 = rel_err(sel_w.reshape(-1, 12)[ok64], ref64[ok64][:, :12], 12)
-        print("config 5 (%d records over %d ticks): vs qpOASES worst %.3e median %.3e; fp32 kernel vs fp64-assembly oracle worst %.3e median %.3e"
-              % (len(recs), len(tick_idx), e32.max(), np.median(e32), e64.max(), np.median(e64)))
-        assert e32.max() < 1e-4 and np.median(e32) < 1e-5
-        assert e64.max() < 2e-3 and np.median(e64) < 1e-4
+    setup = oracle.make_setup(N)
+    ref, info = reference_solve(oracle, recs, setup)
+    ok = info[:, 0] == 0
+    e32 = rel_err(sel_w.reshape(-1, 12)[ok], ref[ok][:, :12], 12)
+    ref64, info64 = reference_solve(oracle, recs, setup, assembly_fp64=True)
+    ok64 = ok & (info64[:, 0] == 0)
+    e64 = rel_err(sel_w.reshape(-1, 12)[ok64], ref64[ok64][:, :12], 12)
+    print("config 5 (%d records over %d ticks): vs qpOASES worst %.3e median %.3e; fp32 kernel vs fp64-assembly oracle worst %.3e median %.3e"
+          % (len(recs), len(tick_idx), e32.max(), np.median(e32), e64.max(), np.median(e64)))
+    assert e32.max() < 1e-4 and np.median(e32) < 1e-5
+    assert e64.max() < 2e-3 and np.median(e64) < 1e-4
     assert (lo["ticks"] == T).all() and lo["failures"].sum() == 0, lo["failures"].sum()
     assert np.isfinite(st["position"]).all()
     assert (np.abs(st["position"][:, 2] - 0.56) < 0.04).all() and (np.abs(st["rpy"][:, :2]) < 0.08).all()
